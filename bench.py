@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
     python bench.py --impl reference --gpus N --steps K ...  # the reference algorithm on host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as .npy
 
 A "step" is one pass of the hot path (the 3-iteration point_flow loop, reference
 pointmvsnet/model.py:297-303) over one reference view per GPU; metric = PointFlow
@@ -25,6 +26,7 @@ import torch
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the benchmark leaves the source tree as it found it (no __pycache__)
 
 CONFIGS = {
     # name: (H, W, V, D)   V counts the reference view (dataset.py:84): "3 src views" = V 4
@@ -72,6 +74,35 @@ def dist_env():
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     return rank, world, local
+
+
+DUMP_LIMIT_BYTES = 64 * 1000 * 1000
+
+
+def pass_outputs(outs, prefix=""):
+    """[(depth, prob)] per iteration of one pass -> {name: tensor} under the reference's prediction names
+    (flow1, flow1_prob, ..., model.py:297-303)."""
+    arrays = {}
+    for i, (depth, prob) in enumerate(outs):
+        arrays["%sflow%d" % (prefix, i + 1)] = depth
+        arrays["%sflow%d_prob" % (prefix, i + 1)] = prob
+    return arrays
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes {name: tensor} as <out_dir>/<name>.npy in float32.  When the arrays hold more than `limit` bytes in
+    all, each one is cut to the same fraction of its elements: a sample drawn with a fixed seed, flattened, in
+    ascending element order, so that two runs with the same arguments write the same positions."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    host = {k: v.detach().float().cpu() for k, v in arrays.items()}
+    total = sum(t.numel() * 4 for t in host.values())
+    frac = min(1.0, (limit - 256 * len(host)) / max(total, 1))  # 256 B per file for the .npy header
+    for name, t in host.items():
+        if frac < 1.0:
+            keep = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:int(t.numel() * frac)]
+            t = t.reshape(-1)[keep.sort().values]
+        np.save(os.path.join(out_dir, name + ".npy"), t.numpy())
 
 
 # --------------------------------------------------------------------------------------
@@ -366,6 +397,14 @@ def run_ours(args):
     clk_p, clk_f = sample_clocks_start(local) if rank == 0 else (None, None)
     total_ms = timed(args.steps, step)
     clocks = sample_clocks_stop(clk_p, clk_f) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results: every view's pass outputs, and with several ranks the gathered depth maps
+        arrays = {}
+        for g, pipe in enumerate(set_a):
+            arrays.update(pass_outputs(pipe.outs, "view%d_" % g))
+        for r, t in enumerate(gathered or []):
+            arrays["rank%d_final_depth" % r] = t
+        dump_outputs(args.dump_outputs, arrays)
     ms_per_step = total_ms / args.steps
     value = world * G * n_iter / (ms_per_step / 1e3)
 
@@ -655,6 +694,9 @@ def run_subcloud(args):
     clk_p, clk_f = sample_clocks_start(local) if rank == 0 else (None, None)
     ms = timed(args.steps, False)
     clocks = sample_clocks_stop(clk_p, clk_f) if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # the pass returns the final depth map (the probabilities of other ranks' sub-clouds are not gathered)
+        dump_outputs(args.dump_outputs, {"flow%d" % n_iter: outs[-1][0]})
     e2e_ms = timed(args.steps, True)
     line = None
     if rank == 0:
@@ -717,10 +759,12 @@ def run_oplevel(args):
     for _ in range(args.steps):
         flush.zero_()
         t0.record()
-        step()
+        outs = step()
         t1.record()
         torch.cuda.synchronize(dev)
         total += t0.elapsed_time(t1)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, pass_outputs(outs))
     ms = total / args.steps
     return json.dumps({
         "metric": METRIC, "value": round(len(IMG_SCALES) / (ms / 1e3), 2), "unit": "iters/s", "n_gpus": 1,
@@ -767,7 +811,15 @@ def main():
     ap.add_argument("--parallel", default="views", choices=["views", "subcloud"],
                     help="views: whole reference views per GPU (throughput, default); subcloud: all GPUs refine ONE "
                          "view, iterations 2/3 split by sub-cloud (BASELINE C5, latency)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32, at "
+                         "most 64 MB in all; a fixed, seeded sample of each array beyond that); the inputs depend "
+                         "only on the arguments, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

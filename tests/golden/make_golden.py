@@ -1,10 +1,10 @@
 #!/usr/bin/env python
 """Generate the golden vectors under tests/golden/ by running the REFERENCE'S OWN
-PYTHON (imported from /root/reference, nothing copied) on CPU.
+PYTHON (imported from a PointMVSNet checkout, nothing copied) on CPU.
 
-Run once in the build container (``python tests/golden/make_golden.py``); the
-resulting .npz files are committed because /root/reference does not exist on the
-GPU box.  The reference is executed with exactly the three adjustments SURVEY.md
+Run once with the checkout at hand (``python tests/golden/make_golden.py <checkout>``); the
+resulting .npz files are committed so that the tests need no reference checkout.
+The reference is executed with exactly the three adjustments SURVEY.md
 section 8c documents, all applied from outside by monkey-patching:
 
   1. ``F.grid_sample`` is called with ``align_corners=True`` (PyTorch 1.0.1
@@ -19,7 +19,8 @@ Files written:
   flow_weights.npz      hot-path weights of outputs/dtu_wde3/model_pretrained.pth
   fetch_known_answer.npz the reference's own known-answer test (feature_fetcher.py:63-97)
   gather_knn.npz        the reference's own gather test (gather_knn.py:27-56), fwd + bwd
-  stages_small.npz      per-stage tensors captured from a real forward (64x128 image)
+  stages_small.npz      per-stage tensors captured from a real forward (64x128 image),
+                        the second EdgeConv's output at the sampled points `ec1_points`
   pass_small.npz        pyramids + coarse depth -> flow1..3, flow{1..3}_prob of that forward
 """
 import os
@@ -30,7 +31,9 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-REF = "/root/reference"
+if len(sys.argv) != 2:
+    sys.exit("usage: make_golden.py <PointMVSNet checkout>")
+REF = os.path.abspath(sys.argv[1])
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, REF)
 sys.path.insert(0, os.path.dirname(os.path.dirname(HERE)))
@@ -212,8 +215,12 @@ def gen_forward(sd):
     # reference feeds to VolumeConv (model.py:113-115)
     save("coarse_small.npz", features=torch.stack(cap["coarse"], dim=1), cams=cams,
          cost_planes=cap["cost"][0][:, :, ::6].contiguous(), plane_stride=np.array(6))
-    # per-stage tensors: iteration 1 (one cloud) and the first sub-cloud of iteration 2
-    st = {}
+    # per-stage tensors: iteration 1 (one cloud) and the first sub-cloud of iteration 2.  The second EdgeConv's
+    # output is kept at a fixed eighth of the points (`ec1_points`) so that the file stays under 1 MB; every other
+    # tensor is stored whole.
+    n_points = cap["knn"][0][1].shape[1]
+    pts = np.sort(np.random.default_rng(0).choice(n_points, n_points // 8, replace=False))
+    st = {"ec1_points": pts}
     for tag, call in (("it1", 0), ("it2", 1)):
         xyz, idx = cap["knn"][call]
         st[tag + "_xyz"] = xyz
@@ -222,7 +229,7 @@ def gen_forward(sd):
             fin, kin, fout = cap["ec"][l][call]
             if l == 0:
                 st[tag + "_feature"] = fin
-            st[tag + "_ec%d_out" % l] = fout
+            st[tag + "_ec%d_out" % l] = fout[:, :, pts].contiguous() if l == 1 else fout
         st[tag + "_mlp_out"] = cap["mlp"][call][1]
     save("stages_small.npz", **st)
     print("flow1 range", preds["flow1"].min().item(), preds["flow1"].max().item())

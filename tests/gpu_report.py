@@ -115,7 +115,7 @@ def main():
                 m.bn.weight.copy_(params["ec%d_gamma" % l]); m.bn.bias.copy_(params["ec%d_beta" % l])
                 m.to(dev).train()
                 x = m(x, idx)
-                err("%s ec%d" % (tag, l), x, st[tag + "_ec%d_out" % l])
+                err("%s ec%d" % (tag, l), x[:, :, st["ec1_points"]] if l == 1 else x, st[tag + "_ec%d_out" % l])
 
     print("== PointFlow iteration stages vs oracle (golden pass inputs)")
     gp = gold("pass_small.npz")

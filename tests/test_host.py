@@ -262,35 +262,62 @@ def test_bench_per_iteration_grouping():
     assert bench.per_iteration_kernel_ms([("knn3d", 1.0)], 3) is None
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/pointmvsnet"), reason="reference checkout not present")
-def test_unchanged_reference_model_imports_our_operators():
-    """Drop-in check (build container only): with install_as_pointmvsnet(reference_root) the
-    reference's UNCHANGED pointmvsnet/model.py resolves its hot-path imports (model.py:8-12) to
-    this package, and its PointMVSNet owns our EdgeConv modules with checkpoint-compatible names."""
-    code = r"""
-import sys
-sys.path.insert(0, %r)
-import pointmvsnet_b200
-pointmvsnet_b200.install_as_pointmvsnet("/root/reference")
-import pointmvsnet.model as m
-import pointmvsnet_b200.networks as ours
-from pointmvsnet_b200.utils.feature_fetcher import FeatureFetcher
-from pointmvsnet_b200.utils.torch_utils import get_knn_3d
-assert m.get_knn_3d is get_knn_3d
-assert m.FeatureFetcher is FeatureFetcher
-net = m.PointMVSNet()
-assert isinstance(net.flow_edge_conv[0], ours.EdgeConvNoC) and isinstance(net.flow_edge_conv[2], ours.EdgeConv)
-assert isinstance(net.feature_fetcher, FeatureFetcher)
-import torch
-sd = torch.load("/root/reference/outputs/dtu_wde3/model_pretrained.pth", map_location="cpu", weights_only=False)["model"]
-net.load_state_dict({k[7:]: v for k, v in sd.items()})
-from pointmvsnet_b200.point_flow import PointFlow
-pf = PointFlow(flow_edge_conv=net.flow_edge_conv, flow_mlp=net.flow_mlp)  # shares the modules
-assert pf.flow_mlp[1].weight is net.flow_mlp[1].weight
-print("DROPIN-OK")
-""" % ROOT
-    out = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
-    assert "DROPIN-OK" in out.stdout, out.stdout + out.stderr
+def test_unchanged_reference_model_imports_our_operators(tmp_path):
+    """Drop-in check against what the reference's UNCHANGED pointmvsnet/model.py resolved (tests/golden/
+    dropin_model.json, written by tests/golden/make_golden_dropin.py from a checkout and its pretrained checkpoint).
+    install_as_pointmvsnet(reference_root) - here over empty stand-ins of the checkout's modules - and the stub mode
+    without a checkout both hand out our object for every name model.py took from this package (model.py:8-12);
+    the submodules PointMVSNet built from our classes have the checkpoint's layout, and PointFlow builds them under
+    the same names or runs on a model's own modules."""
+    import importlib
+    import json
+    import pointmvsnet_b200
+    from pointmvsnet_b200.point_flow import PointFlow
+    with open(os.path.join(ROOT, "tests", "golden", "dropin_model.json")) as f:
+        g = json.load(f)
+
+    def resolve(path):
+        mod, qual = path.split(":")
+        return getattr(importlib.import_module(mod), qual)
+
+    for name, kind in g["reference_modules"].items():
+        p = tmp_path.joinpath(*name.split("."))
+        if kind == "package":
+            p.mkdir(parents=True, exist_ok=True)
+            (p / "__init__.py").write_text("")
+        else:
+            p.parent.mkdir(parents=True, exist_ok=True)
+            p.with_suffix(".py").write_text("")
+    assert g["imports"]
+
+    def drop_aliases():
+        for k in [k for k in sys.modules if k == "pointmvsnet" or k.startswith("pointmvsnet.")]:
+            del sys.modules[k]
+
+    saved = {k: v for k, v in sys.modules.items() if k == "pointmvsnet" or k.startswith("pointmvsnet.")}
+    saved_path = list(sys.path)
+    try:
+        for root in (str(tmp_path), None):
+            drop_aliases()
+            pointmvsnet_b200.install_as_pointmvsnet(root)
+            for name, rec in g["imports"].items():
+                obj = resolve(rec["object"])
+                for mod in rec["from"]:
+                    assert getattr(importlib.import_module(mod), name, None) is obj, (root, mod, name)
+    finally:
+        drop_aliases()
+        sys.modules.update(saved)
+        sys.path[:] = saved_path
+    pf = PointFlow()
+    own = dict(pf.named_modules())
+    assert g["submodules"]
+    for path, rec in g["submodules"].items():
+        cls = resolve(rec["class"])
+        mod = own[path] if path in own else cls()
+        assert type(mod) is cls, path
+        assert {k: list(v.shape) for k, v in mod.state_dict().items()} == rec["state"], path
+    shared = PointFlow(flow_edge_conv=pf.flow_edge_conv, flow_mlp=pf.flow_mlp)
+    assert shared.flow_mlp[1].weight is pf.flow_mlp[1].weight
 
 
 def test_image_conv_producer_names_layout_and_probability_map():
