@@ -437,12 +437,14 @@ def test_linear_pm_modes_vs_fp64(mode, rtol, cin, cout, rows):
     assert torch.allclose(out_stats[cout:], (want * want).sum(0), rtol=2 * srt + 1e-4)
 
 
-@pytest.mark.parametrize("gemm_opt", [0, 1])
+@pytest.mark.parametrize("gemm_opt", [0, 1, 2])
 @pytest.mark.parametrize("cin,cout,groups,rows", [(64, 64, 3, 1000), (136, 64, 2, 25600), (64, 128, 5, 333),
                                                   (64, 16, 4, 4097), (32, 64, 16, 640), (224, 64, 2, 129)])
 def test_linear_pm_groups_ragged_tiles_both_tcgen05_kernels(gemm_opt, cin, cout, groups, rows):
     """Several BatchNorm groups per launch (per-group input statistics, per-group output sums), row counts that
-    are not multiples of the 128-point tile, for both tensor-core kernels (gemm_tc.cu / gemm_ws.cu), 3xTF32."""
+    are not multiples of the 128-point tile, for both tensor-core kernels (gemm_tc.cu / gemm_ws.cu with register
+    prefetch or cp.async staging), 3xTF32.  cin = 64 also reads x as a slice of wider rows, as the fused iteration
+    reads EdgeConv 2's input: 64 columns at offset 32 of the 224-column EdgeConv concat (ldx = 224)."""
     from pointmvsnet_b200 import _lib
     gen = torch.Generator().manual_seed(cin * 7 + cout + groups)
     x = (torch.randn(groups, rows, cin, generator=gen) * (1 + torch.arange(groups).view(-1, 1, 1))).to(DEV)
@@ -453,13 +455,20 @@ def test_linear_pm_groups_ragged_tiles_both_tcgen05_kernels(gemm_opt, cin, cout,
     in_stats = torch.cat([xs.sum(1), (xs * xs).sum(1)], dim=1).contiguous()  # [groups, 2*cin]
     y = torch.full((groups, rows, cout), float("nan"), device=DEV)
     out_stats = torch.zeros(groups, 2 * cout, device=DEV, dtype=torch.float64)
+    layouts = [(x, cin, 0)]
+    if cin == 64:
+        # large finite values around the slice: a column read outside it changes the result
+        wide = (1e3 * torch.randn(groups, rows, 224, generator=gen)).to(DEV)
+        wide[:, :, 32:96] = x
+        layouts.append((wide, 224, 32))
     old = _lib.get_option("gemm")
     try:
         _lib.set_option("gemm", gemm_opt)
-        for use_bn in (True, False):
+        for (buf, ldx, col), use_bn in [(lay, bn) for lay in layouts for bn in (True, False)]:
             out_stats.zero_()
-            _lib.check(_lib.lib.pmvs_linear_pm(x.data_ptr(), cin, w.data_ptr(), y.data_ptr(), cout, groups, rows, cin,
-                                               cout, in_stats.data_ptr() if use_bn else None,
+            y.fill_(float("nan"))
+            _lib.check(_lib.lib.pmvs_linear_pm(buf.data_ptr() + 4 * col, ldx, w.data_ptr(), y.data_ptr(), cout, groups,
+                                               rows, cin, cout, in_stats.data_ptr() if use_bn else None,
                                                gamma.data_ptr() if use_bn else None, beta.data_ptr() if use_bn else None,
                                                float(rows), 1e-5, out_stats.data_ptr(), _lib.stream_ptr()))
             torch.cuda.synchronize()
@@ -472,7 +481,7 @@ def test_linear_pm_groups_ragged_tiles_both_tcgen05_kernels(gemm_opt, cin, cout,
             want = xn @ w.double().t()
             scale = (xn.abs() @ w.double().abs().t()).clamp(min=1e-6)
             err = ((y.double() - want).abs() / scale).max().item()
-            assert err < 1e-5, (gemm_opt, use_bn, cin, cout, err)
+            assert err < 1e-5, (gemm_opt, use_bn, ldx, cin, cout, err)
             assert torch.allclose(out_stats[:, :cout], want.sum(1), rtol=1e-4, atol=1e-4 * scale.sum(1).max().item())
             assert torch.allclose(out_stats[:, cout:], (want * want).sum(1), rtol=3e-4)
     finally:
@@ -649,8 +658,9 @@ def test_coarse_cost_volume_golden_and_oracle():
 
 
 def test_edgeconv_generic_paths_runtime_k_and_simt_fallback():
-    """K != 16 (runtime-K gather loop), out_channels 16 (contraction falls back to the fp32 SIMT
-    kernel: the tcgen05 path covers N in {16, 64, 128}) and a ragged point count."""
+    """K != 16 (runtime-K gather loop), out_channels 16 (the 16-channel instance of the gather EdgeConv kernels;
+    its contraction, cin 16 -> 2 x 16 = 32 columns, runs on the warp-specialised tcgen05 GEMM, gemm_ws.cu, like
+    the other shapes here) and a ragged point count."""
     from pointmvsnet_b200.networks import EdgeConv, EdgeConvNoC
     gen = torch.Generator().manual_seed(41)
     for cls, cin, cout, K, concat in ((EdgeConv, 16, 16, 8, True), (EdgeConvNoC, 24, 32, 5, False),
